@@ -27,6 +27,9 @@ Timing: CUDA events on the launching stream, barrier + synchronize on both sides
 resident inputs of the default workload (13.4 GB cache + 3.4 GB embeddings per rank) are far larger than the
 126 MB L2, so no explicit L2 flush is needed between iterations (stated in config).  Outside the timed region a
 parity gate re-checks a 1 024-row slice of the timed batch against the CPU oracle (`parity_gate` in the line).
+
+--dump-outputs DIR writes what the last timed `value` step returned (rank 0) as DIR/<name>.npy, so that two
+builds run with the same arguments (and therefore the same seeded inputs) can be compared output for output.
 """
 
 from __future__ import annotations
@@ -41,6 +44,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark may run from a read-only checkout: no bytecode caches in the tree, here or in the CPU-arm workers
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 import torch  # noqa: E402
 
@@ -75,7 +81,55 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-parity-gate", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the last timed step's outputs as DIR/<name>.npy (at most 64 MB in all)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
+
+
+# ------------------------------------------------------------------------------------ output dump
+DUMP_BYTES = 64 << 20
+
+
+def _dump_dtype(t):
+    """float32, or float64 where float32 would not hold the values exactly (float64 data, integers >= 2^24)."""
+    if t.dtype == torch.float64:
+        return torch.float64
+    if t.dtype.is_floating_point or t.numel() == 0:
+        return torch.float32
+    return torch.float32 if int(t.abs().max()) < 2 ** 24 else torch.float64
+
+
+def dump_outputs(res, out_dir, budget=DUMP_BYTES):
+    """Write every tensor (and scalar) of a step's result as out_dir/<name>.npy.  When the whole set exceeds
+    `budget`, the arrays that share the batch (leading) dimension are restricted to a fixed seeded sample of
+    rows, the same rows for every array, and the sorted row indices go to out_dir/sample_rows.npy."""
+    import numpy as np
+
+    arrays = {}
+    for k, v in res.items():
+        if isinstance(v, torch.Tensor):
+            arrays[k] = v.detach()
+        elif isinstance(v, (int, float)) and not isinstance(v, bool):
+            arrays[k] = torch.tensor(float(v), dtype=torch.float64)
+    arrays = {k: v.to(_dump_dtype(v)) for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in arrays.values())
+    if total > budget:
+        rows = max(v.shape[0] for v in arrays.values() if v.dim() > 0)
+        batched = [k for k, v in arrays.items() if v.dim() > 0 and v.shape[0] == rows]
+        fixed = total - sum(arrays[k].numel() * arrays[k].element_size() for k in batched)
+        per_row = sum(arrays[k][0].numel() * arrays[k].element_size() for k in batched)
+        keep = (budget - fixed - rows * 8) // per_row
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        for k in batched:
+            arrays[k] = arrays[k][idx.to(arrays[k].device)]
+        arrays["sample_rows"] = idx.to(torch.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.cpu().numpy())
+    return sorted(arrays)
 
 
 # ------------------------------------------------------------------------------------ clocks
@@ -459,6 +513,7 @@ def run_ours(args, wl):
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop(t_mark0, t_mark1) if sampler else None
     n_launch = native.LAUNCH_COUNT - launch0
+    dumped = dump_outputs(res, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     sel = torch.tensor([sel_per_step_rank], dtype=torch.float64, device=dev)
     if world > 1:
@@ -552,6 +607,8 @@ def run_ours(args, wl):
         "clocks": clocks, "e2e": e2e, "gpu_launches": n_launch, "roofline": roofline, "cpu_baseline": cpu_baseline,
         "selections_per_step": sel_total_per_step, "parity_gate": gate,
     }
+    if dumped is not None:
+        line["dumped_outputs"] = {"dir": args.dump_outputs, "arrays": dumped}
     if kind == "train":
         line["train_step"] = {"sampling_phase_ms": k_ms_avg, "micro_batch": args.micro_batch,
                               "chunks": res.get("chunks"), "loss": float(res["loss"]),

@@ -8,10 +8,10 @@ paths.  ``oracle/_ref/`` is git-ignored (reference sources never enter the histo
 gpurun-ignored, so it travels to the GPU box with the snapshot like a built ``.so`` does.
 ``__graft_entry__.build()`` calls :func:`make` whenever ``/root/reference`` is present.
 
-Consumers (all test / bench infrastructure; the product package never imports ``oracle/``):
+Consumers (bench / fixture infrastructure; the product package never imports ``oracle/``):
   * ``bench.py --impl reference`` and ``bench.py``'s ``cpu_baseline`` leg  (kind "reference")
-  * ``tests/test_gpu_dropin.py``   -- the reference's own loop driving the CUDA drop-ins
-  * ``tests/test_oracle_vs_reference.py``
+  * ``tests/golden/make_golden.py``, which records what the tests compare against; the tests themselves
+    read only the recorded fixtures
 
     python oracle/make_ref.py            # (re)stage
     python oracle/make_ref.py --check    # verify staged files are byte-identical to the source

@@ -30,8 +30,8 @@ module is computed by reference code + PyTorch.
 ``/root/reference`` does not exist on the GPU box.  ``oracle/make_ref.py`` (called by
 ``__graft_entry__.build()`` in the build container) stages the same unmodified files under the
 git-ignored ``oracle/_ref/``, which travels with the snapshot; this module uses
-``/root/reference`` when present and ``oracle/_ref`` otherwise.  Tests that need it skip when
-neither exists.
+the reference tree when present and ``oracle/_ref`` otherwise.  No test needs it: the tests compare
+against fixtures recorded through it (tests/golden/make_golden.py).
 """
 
 from __future__ import annotations

@@ -94,3 +94,44 @@ def name_seeded_weights(state_dict, seed):
         else:
             new[k] = 0.1 * u
     return new
+
+
+def seeded_weights_from_meta(meta, seed):
+    """name_seeded_weights of a state_dict described by tests/golden/make_golden.py::weight_meta (names, shapes and
+    float flags as JSON)."""
+    import json
+
+    spec = json.loads(str(meta))
+    return name_seeded_weights({k: torch.zeros(shape, dtype=torch.float32 if is_float else torch.int64)
+                                for k, (shape, is_float) in spec.items()}, int(seed))
+
+
+def seeded_instances(spec, crcs):
+    """The instances tests/golden/make_golden.py::seeded_instances drew from the reference's generator, regenerated
+    by the project's generator under the same torch seed; every array must match the reference's CRC-32."""
+    import json
+    import zlib
+
+    from rl4co_b200.envs import get_env
+
+    spec = json.loads(str(spec))
+    torch.manual_seed(spec["seed"])
+    td = get_env(spec["env"], generator_params=dict(num_loc=spec["n"])).generator(spec["batch"])
+    inst = {k: td[k] for k in td.keys()}
+    assert set(inst) == set(crcs), (sorted(inst), sorted(crcs))
+    for k, v in inst.items():
+        assert zlib.crc32(v.numpy().tobytes()) == int(crcs[k]), f"regenerated {spec['env']} instances differ in {k}"
+    return inst
+
+
+def golden_case(z, tag):
+    """One case `tag/...` of a multi-case fixture as tensors: (instances, outputs, weights); instances and weights
+    are regenerated from their seeds when the fixture holds only those."""
+    pre = tag + "/"
+    arr = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+    outs = {k: torch.from_numpy(v.astype(np.int64) if v.dtype == np.uint8 else v) for k, v in arr.items()
+            if "::" not in k and v.dtype.kind != "U"}
+    inst = seeded_instances(arr["gen"], {k[5:]: v for k, v in arr.items() if k.startswith("crc::")}) \
+        if "gen" in arr else None
+    W = seeded_weights_from_meta(arr["w_meta"], arr["weight_seed"]) if "w_meta" in arr else None
+    return inst, outs, W

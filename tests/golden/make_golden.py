@@ -16,8 +16,10 @@ batchify / dihedral-8 layout conventions.
 
 from __future__ import annotations
 
+import json
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
@@ -365,8 +367,185 @@ def layout_fixture():
                 tsp_num_starts=np.int64(env.get_num_starts(tdx)), cvrp_num_starts=np.int64(envc.get_num_starts(tdc)))
 
 
+def weight_meta(module):
+    """Names / shapes / float flags of a state_dict: with the weight seed this is all a consumer needs to rebuild
+    name_seeded_weights (tests/conftest.py::seeded_weights_from_meta)."""
+    return np.array(json.dumps({k: [list(v.shape), bool(v.dtype.is_floating_point)]
+                                for k, v in module.state_dict().items()}))
+
+
+def seeded_instances(out, tag, name, n, batch, seed):
+    """The reference generator's instances after torch.manual_seed(seed): a consumer regenerates them with the
+    project's generator (tests/conftest.py::golden_case) and checks them against the stored CRC-32 of each array."""
+    torch.manual_seed(seed)
+    env = make_env(name, n)
+    td0 = env.generator(batch_size=[batch])
+    out[f"{tag}/gen"] = np.array(json.dumps({"env": name, "n": n, "batch": batch, "seed": seed}))
+    out.update({f"{tag}/crc::{k}": np.int64(zlib.crc32(npy(td0[k]).tobytes())) for k in td0.keys()})
+    return env, td0
+
+
+def policy_case(out, tag, name, n, batch, seed, layers, decode_type, sample_seed=None, phase="test", evaluate=False,
+                step_rows=0, **kw):
+    """One reference policy forward on name-seeded weights: seeded instances, actions, log-likelihood, reward, the
+    per-step log-probs of the first `step_rows` trajectories (and, with `evaluate`, the teacher-forced pass on its
+    own actions).  `sample_seed` seeds the torch generator right before the forward, so a consumer regenerates the
+    Exp(1) draws torch.multinomial took."""
+    env, td0 = seeded_instances(out, tag, name, n, batch, seed)
+    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=layers).eval()
+    name_seeded_weights(pol, seed)
+    with torch.inference_mode():
+        if sample_seed is not None:
+            torch.manual_seed(sample_seed)
+        o = pol(env.reset(td0.clone()), env, phase=phase, decode_type=decode_type, return_sum_log_likelihood=False, **kw)
+        if evaluate:
+            e = pol(env.reset(td0.clone()), env, phase=phase, actions=o["actions"], return_sum_log_likelihood=False)
+            out.update({f"{tag}/eval_ll": npy(e["log_likelihood"].sum(-1)), f"{tag}/eval_reward": npy(e["reward"]),
+                        f"{tag}/eval_logprobs": npy(e["log_likelihood"][:step_rows])})
+    acts = o["actions"]
+    out.update({f"{tag}/actions": npy(acts).astype(np.uint8) if acts.max() < 256 else npy(acts),
+                f"{tag}/ll": npy(o["log_likelihood"].sum(-1)), f"{tag}/reward": npy(o["reward"]),
+                f"{tag}/w_meta": weight_meta(pol), f"{tag}/weight_seed": np.int64(seed)})
+    if step_rows:
+        out[f"{tag}/logprobs"] = npy(o["log_likelihood"][:step_rows])
+
+
+def ref_policy_fixture():
+    """tests/test_oracle_vs_reference.py: the reference's policy forward over decode types, filters, beam search and
+    the sibling envs; its generator; process_logits with top-k / top-p."""
+    out = {}
+    for name, n in (("tsp", 20), ("cvrp", 20), ("tsp", 37), ("cvrp", 33)):
+        for dt in ("greedy", "sampling", "multistart_greedy", "multistart_sampling"):
+            policy_case(out, f"fwd_{name}{n}_{dt}", name, n, 6, 1000 + n, 2, dt, sample_seed=5)
+    for name in ("tsp", "cvrp"):
+        policy_case(out, f"multinomial_{name}", name, 20, 32, 3, 1, "sampling", sample_seed=7, phase="train")
+        policy_case(out, f"filters_{name}", name, 20, 16, 21, 1, "sampling", sample_seed=9, phase="train", top_k=5,
+                    top_p=0.9)
+    for name, n in (("tsp", 12), ("cvrp", 11)):
+        for bw, sb in ((3, True), (4, False), (None, True)):
+            kw = {} if bw is None else {"beam_width": bw}
+            policy_case(out, f"beam_{name}{n}_{bw}_{sb}", name, n, 5, 300 + n, 1, "beam_search", select_best=sb, **kw)
+    for name, n in (("op", 20), ("op", 33), ("pctsp", 20), ("pctsp", 41), ("sdvrp", 20)):
+        for dt in ("greedy", "sampling"):
+            policy_case(out, f"sibling_{name}{n}_{dt}", name, n, 8, 2000 + n, 2, dt, sample_seed=5)
+    for name, n in (("tsp", 50), ("cvrp", 50), ("cvrp", 100)):
+        env = make_env(name, n)
+        torch.manual_seed(1234)
+        td = env.generator(batch_size=[5])
+        out.update({f"gen_{name}{n}/{k}": npy(td[k]) for k in td.keys()})
+    for top_k, top_p in ((3, 0.0), (0, 0.6), (4, 0.8), (50, 0.0), (0, 1.0)):
+        torch.manual_seed(11 + top_k)
+        logits = torch.randn(32, 20) * 2
+        logits[:, 7] = logits[:, 3]
+        mask = torch.rand(32, 20) > 0.4
+        mask[:, 1] = True
+        want = ref.decoding.process_logits(logits.clone(), mask, temperature=1.3, top_p=top_p, top_k=top_k,
+                                           tanh_clipping=10.0)
+        out.update({f"process_{top_k}_{top_p}/logits": npy(logits), f"process_{top_k}_{top_p}/mask": npy(mask),
+                    f"process_{top_k}_{top_p}/want": npy(want)})
+    return out
+
+
+def ref_baselines_fixture():
+    """tests/test_baselines_cpu.py: the reference's REINFORCE baselines (models/rl/reinforce/baselines.py) on the
+    test's fake policy / env."""
+    import copy
+    import importlib
+
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_baselines_cpu import ROLLOUT_CANDIDATES, CriticPolicy, FakeEnv, FakePolicy, baseline_inputs
+
+    class RefDataset(torch.utils.data.Dataset):
+        """the reference's DataLoader path needs a dataset with `collate_fn` (data/dataset.py:41-78)."""
+
+        def __init__(self, ds):
+            self.ds, self.collate_fn = ds, ds.collate_fn
+
+        def __len__(self):
+            return len(self.ds)
+
+        def __getitem__(self, i):
+            return self.ds[i]
+
+    class RefEnv(FakeEnv):
+        def dataset(self, batch_size=[], **kw):
+            return RefDataset(super().dataset(batch_size))
+
+    bl = importlib.import_module("rl4co.models.rl.reinforce.baselines")
+    inp = baseline_inputs()
+    out = {}
+    for i, cand in enumerate(ROLLOUT_CANDIDATES):
+        theirs = bl.RolloutBaseline(bl_alpha=0.05)
+        theirs.setup(FakePolicy(0.0), RefEnv(), batch_size=16, device="cpu", dataset_size=64)
+        out[f"rollout{i}/setup_mean"], out[f"rollout{i}/bl_vals"] = npy(float(theirs.mean)), npy(theirs.bl_vals)
+        theirs.epoch_callback(copy.deepcopy(FakePolicy(**cand)), RefEnv(), batch_size=16, device="cpu", epoch=0,
+                              dataset_size=64)
+        out[f"rollout{i}/mean"], out[f"rollout{i}/bias"] = npy(float(theirs.mean)), npy(float(theirs.policy.bias))
+        td = TensorDict({"x": torch.from_numpy(inp["rollout_x"])}, batch_size=[7])
+        out[f"rollout{i}/eval"] = npy(theirs.eval(td, None, RefEnv())[0])
+    theirs = bl.get_reinforce_baseline("rollout", n_epochs=2, exp_beta=0.8)
+    theirs.setup(FakePolicy(0.1), RefEnv(), batch_size=16, device="cpu", dataset_size=32)
+    vals, alphas = [], []
+    for epoch in range(3):
+        for j in range(2):
+            td = TensorDict({"x": torch.from_numpy(inp["warmup_x"][epoch, j])}, batch_size=[9])
+            v, l = theirs.eval(td, torch.from_numpy(inp["warmup_reward"][epoch, j]), RefEnv())
+            assert float(l) == 0.0
+            vals.append(npy(torch.as_tensor(v).float().expand(9)))
+        theirs.epoch_callback(FakePolicy(0.1), RefEnv(), batch_size=16, device="cpu", epoch=epoch, dataset_size=32)
+        alphas.append(float(theirs.alpha))
+    out["warmup/values"], out["warmup/alpha"] = np.stack(vals), np.array(alphas)
+    torch.manual_seed(1)
+    pol = CriticPolicy()
+    theirs = bl.CriticBaseline()
+    torch.manual_seed(2)
+    theirs.setup(pol, FakeEnv())
+    v, l = theirs.eval(TensorDict({"locs": torch.from_numpy(inp["critic_locs"])}, batch_size=[6]),
+                       torch.from_numpy(inp["critic_reward"]))
+    out["critic/keys"] = np.array(list(theirs.critic.state_dict().keys()))
+    out["critic/value"], out["critic/loss"] = npy(v), npy(l)
+    names = ("no", "shared", "exponential", "mean", "critic", "rollout_only", "rollout", "warmup")
+    out["registry/names"] = np.array(names)
+    out["registry/types"] = np.array([type(bl.get_reinforce_baseline(n)).__name__ for n in names])
+    return out
+
+
+def ref_datasets_fixture():
+    """tests/test_host_cpu.py: the reference's numpy-seeded validation / test sets (data/generate_data.py)."""
+    import importlib
+
+    G = importlib.import_module("rl4co.data.generate_data")
+    out = {}
+    for prob, gs, seed, name in (("tsp", 20, 4321, "val"), ("vrp", 50, 1234, "test")):
+        np.random.seed(seed)
+        out.update({f"{prob}{gs}_{name}/{k}": v for k, v in G.generate_env_data(prob, 16, gs, None).items()})
+    return out
+
+
+def dropin_fixture():
+    """tests/test_gpu_dropin.py and the sibling envs' drop-in tests: what the reference's own loop computes, to be
+    matched by the CUDA env / decoder -- random-policy MDP traces (utils/decoding.py:85-106) and policy forwards
+    on name-seeded weights (sampling: Exp(1) draws regenerated from the seed)."""
+    out = {}
+    for name, n in (("tsp", 20), ("cvrp", 20), ("tsp", 50), ("cvrp", 50)):
+        seeded_instances(out, f"env_{name}{n}", name, n, 64, 11)  # the instances env_fixture draws first
+        trace = env_fixture(name, n, 64, 11)
+        out.update({f"env_{name}{n}/{k}": v for k, v in trace.items() if not k.startswith("inst::")})
+        for dt in ("greedy", "sampling", "multistart_greedy"):
+            policy_case(out, f"fwd_{name}{n}_{dt}", name, n, 32, 13, 2, dt, sample_seed=3,
+                        evaluate="multistart" not in dt, step_rows=8)
+    policy_case(out, "op20_sampling", "op", 20, 64, 3, 1, "sampling", sample_seed=11, phase="train", step_rows=8)
+    policy_case(out, "pctsp20_sampling", "pctsp", 20, 64, 3, 1, "sampling", sample_seed=11, phase="train", step_rows=8)
+    policy_case(out, "sdvrp20_greedy", "sdvrp", 20, 32, 3, 1, "greedy", step_rows=8)
+    return out
+
+
 def main():
     jobs = {
+        "ref_policy": ref_policy_fixture,
+        "ref_baselines": ref_baselines_fixture,
+        "ref_datasets": ref_datasets_fixture,
+        "dropin": dropin_fixture,
         "env_tsp20": lambda: env_fixture("tsp", 20, 16, 100),
         "env_tsp50": lambda: env_fixture("tsp", 50, 8, 101),
         "env_cvrp20": lambda: env_fixture("cvrp", 20, 16, 102),

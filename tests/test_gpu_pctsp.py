@@ -190,39 +190,15 @@ def test_pctsp_fused_equals_stepping():
 
 
 def test_pctsp_under_the_reference_loop():
-    """Drop-in: the reference's own ConstructivePolicy.forward + DecodingStrategy (unmodified files, staged under
-    oracle/_ref) drive FusedPCTSPEnv and the CUDA decoder; equal to the pure reference on the same weights, instances and
-    sampling seed."""
-    import importlib
+    """Drop-in: the reference's own ConstructivePolicy.forward + DecodingStrategy on its PCTSP env, as recorded in
+    tests/golden/dropin.npz, reproduced by FusedPCTSPEnv and the CUDA decoder on the same weights, instances and
+    sampling draws."""
+    import os
 
-    from oracle import ref_standin
+    import numpy as np
 
-    if not ref_standin.reference_available():
-        pytest.skip("no reference tree (oracle/_ref not staged)")
-    ref = ref_standin.load()
-    from rl4co_b200.decoder import FusedAttentionModelDecoder
-    from rl4co_b200.envs import get_env
+    from test_gpu_dropin import check_forward_against_reference
 
-    PCTSPEnv = importlib.import_module("rl4co.envs.routing.pctsp.env").PCTSPEnv
-    env_ref = PCTSPEnv(generator_params=dict(num_loc=20), check_solution=True)
-    env_fused = get_env("pctsp", generator_params=dict(num_loc=20), check_solution=True)
-    torch.manual_seed(3)
-    pure = ref.AttentionModelPolicy(env_name="pctsp", num_encoder_layers=1).to(DEV).eval()
-    dec = FusedAttentionModelDecoder(env_name="pctsp")
-    dec.cache_gemm = "cublas"
-    mixed = ref.AttentionModelPolicy(env_name="pctsp", num_encoder_layers=1, decoder=dec)
-    res = mixed.load_state_dict(pure.state_dict())
-    assert not res.missing_keys and not res.unexpected_keys
-    mixed = mixed.to(DEV).eval()
-    td0 = env_ref.generator(batch_size=[64]).to(DEV)
-    with torch.inference_mode():
-        torch.manual_seed(11)
-        a = pure(env_ref.reset(td0.clone()), env_ref, phase="train", decode_type="sampling", return_sum_log_likelihood=False)
-        torch.manual_seed(11)
-        b = mixed(env_fused.reset(td0.clone()), env_fused, phase="train", decode_type="sampling",
-                  return_sum_log_likelihood=False)
-    same = (a["actions"] == b["actions"]).all(1) if a["actions"].shape == b["actions"].shape else None
-    assert same is not None and same.float().mean() >= 0.9
-    assert (a["actions"] != 0).any(1).float().mean() > 0.5  # the sampled tours are not trivial
-    torch.testing.assert_close(b["log_likelihood"][same], a["log_likelihood"][same], rtol=RTOL, atol=ATOL_LP)
-    torch.testing.assert_close(b["reward"][same], a["reward"][same], rtol=RTOL, atol=1e-6)
+    ref = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dropin.npz"))
+    *_, want = check_forward_against_reference(ref, "pctsp20_sampling", "pctsp", 20, 1, "sampling", sample_seed=11, phase="train")
+    assert (want["actions"] != 0).any(1).float().mean() > 0.5  # the sampled tours are not trivial

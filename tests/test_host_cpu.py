@@ -335,27 +335,23 @@ def test_bench_reference_arm_line_schema():
 def test_seeded_dataset_generation_matches_reference(tmp_path):
     """data/generate_data.py:37-76,213-317: the numpy-seeded validation / test sets are bit-identical to the
     reference's; `env.dataset(phase=...)` loads them (SURVEY.md 8f-3)."""
-    import importlib
-
     import numpy as np
 
-    from oracle import ref_standin
     from rl4co_b200 import data as D
     from rl4co_b200.envs import get_env
 
     files = D.generate_default_datasets(str(tmp_path), dataset_size=16, graph_sizes=(20, 50))
     assert len(files) == 8 and all(os.path.isfile(f) for f in files)
     assert os.path.basename(files[0]) == "tsp20_val_seed4321.npz" and os.path.basename(files[-1]) == "vrp50_test_seed1234.npz"
-    if ref_standin.reference_available():
-        ref_standin.install()
-        G = importlib.import_module("rl4co.data.generate_data")
-        for prob, gs, seed, name in (("tsp", 20, 4321, "val"), ("vrp", 50, 1234, "test")):
-            np.random.seed(seed)
-            want = G.generate_env_data(prob, 16, gs, None)
-            got = np.load(D.dataset_filename(str(tmp_path), prob, gs, name, seed))
-            assert set(got.files) == set(want.keys())
-            for k in want:
-                assert np.array_equal(got[k], want[k]), (prob, k)
+    # the reference's own sets, recorded by tests/golden/make_golden.py (ref_datasets.npz)
+    ref = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_datasets.npz"))
+    for prob, gs, seed, name in (("tsp", 20, 4321, "val"), ("vrp", 50, 1234, "test")):
+        prefix = f"{prob}{gs}_{name}/"
+        want = {k[len(prefix):]: ref[k] for k in ref.files if k.startswith(prefix)}
+        got = np.load(D.dataset_filename(str(tmp_path), prob, gs, name, seed))
+        assert want and set(got.files) == set(want)
+        for k in want:
+            assert np.array_equal(got[k], want[k]), (prob, k)
     env = get_env("cvrp", generator_params=dict(num_loc=20), data_dir=str(tmp_path), val_file="vrp/vrp20_val_seed4321.npz")
     ds = env.dataset(phase="val")
     assert len(ds) == 16

@@ -1,146 +1,97 @@
-"""CPU, build container only: re-run the LIVE reference (unmodified files from /root/reference
-through oracle/ref_standin.py) against oracle/am_rollout_oracle.py on fresh seeds.
-Skipped where /root/reference does not exist (the GPU box)."""
+"""CPU: oracle/am_rollout_oracle.py against what the unmodified reference computed on the same instances, weights
+and seeds, recorded in tests/golden/ref_policy.npz (tests/golden/make_golden.py): policy forwards over every decode
+type, top-k / top-p filters, beam search, the sibling envs, the instance generator."""
 
+import os
+
+import numpy as np
 import pytest
 import torch
 
+from conftest import golden_case
 from oracle import am_rollout_oracle as O
-from oracle import ref_standin
-
-pytestmark = pytest.mark.skipif(not ref_standin.reference_available(), reason="/root/reference not present")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    return ref_standin.load()
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_policy.npz"))
 
 
 @pytest.mark.parametrize("name,n", [("tsp", 20), ("cvrp", 20), ("tsp", 37), ("cvrp", 33)])
 @pytest.mark.parametrize("decode_type", ["greedy", "sampling", "multistart_greedy", "multistart_sampling"])
 def test_policy_forward_matches_reference(ref, name, n, decode_type):
-    torch.manual_seed(1000 + n)
-    Env = ref.TSPEnv if name == "tsp" else ref.CVRPEnv
-    env = Env(generator_params=dict(num_loc=n), check_solution=True)
-    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=2).eval()
-    W = {k: v.detach().clone() for k, v in pol.state_dict().items()}
-    td0 = env.generator(batch_size=[6])
-    inst = {k: td0[k].clone() for k in td0.keys()}
+    inst, want, W = golden_case(ref, f"fwd_{name}{n}_{decode_type}")
     with torch.inference_mode():
-        td = env.reset(td0.clone())
-        torch.manual_seed(5)
-        out = pol(td.clone(), env, phase="test", decode_type=decode_type)
         torch.manual_seed(5)
         o = O.policy_forward(W, name, inst, decode_type=decode_type, num_layers=2)
-    assert torch.equal(out["actions"], o["actions"])
-    torch.testing.assert_close(out["reward"], o["reward"], rtol=1e-6, atol=0)
-    torch.testing.assert_close(out["log_likelihood"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
+    assert torch.equal(want["actions"], o["actions"])
+    torch.testing.assert_close(want["reward"], o["reward"], rtol=1e-6, atol=0)
+    torch.testing.assert_close(want["ll"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
 
 
 @pytest.mark.parametrize("name", ["tsp", "cvrp"])
 def test_multinomial_is_argmax_p_over_exp_noise(ref, name):
     """The recorded-noise protocol used for sampling parity: torch.multinomial(p,1) consumes
     exactly one empty_like(p).exponential_(1) draw per step."""
-    torch.manual_seed(3)
-    Env = ref.TSPEnv if name == "tsp" else ref.CVRPEnv
-    env = Env(generator_params=dict(num_loc=20), check_solution=True)
-    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=1).eval()
-    W = {k: v.detach().clone() for k, v in pol.state_dict().items()}
-    td0 = env.generator(batch_size=[32])
-    inst = {k: td0[k].clone() for k in td0.keys()}
+    inst, want, W = golden_case(ref, f"multinomial_{name}")
     with torch.inference_mode():
-        torch.manual_seed(7)
-        out = pol(env.reset(td0.clone()), env, phase="train", decode_type="sampling")
         torch.manual_seed(7)
         o = O.policy_forward(W, name, inst, decode_type="sampling", num_layers=1,
                              noise=lambda t, shape: torch.empty(shape).exponential_(1))
-    assert torch.equal(out["actions"], o["actions"])
+    assert torch.equal(want["actions"], o["actions"])
 
 
 @pytest.mark.parametrize("top_k,top_p", [(3, 0.0), (0, 0.6), (4, 0.8), (50, 0.0), (0, 1.0)])
 def test_top_k_top_p_process_logits_matches_reference(ref, top_k, top_p):
     """utils/decoding.py:109-188 with the filters on, bit for bit (same torch ops in the same order)."""
-    torch.manual_seed(11 + top_k)
-    logits = torch.randn(32, 20) * 2
-    logits[:, 7] = logits[:, 3]
-    mask = torch.rand(32, 20) > 0.4
-    mask[:, 1] = True
-    want = ref.decoding.process_logits(logits.clone(), mask, temperature=1.3, top_p=top_p, top_k=top_k, tanh_clipping=10.0)
-    got = O.process_logits(logits.clone(), mask, temperature=1.3, tanh_clipping=10.0, top_k=top_k, top_p=top_p)
-    assert torch.equal(want, got)
+    _, case, _ = golden_case(ref, f"process_{top_k}_{top_p}")
+    got = O.process_logits(case["logits"].clone(), case["mask"], temperature=1.3, tanh_clipping=10.0, top_k=top_k,
+                           top_p=top_p)
+    assert torch.equal(case["want"], got)
 
 
 @pytest.mark.parametrize("name", ["tsp", "cvrp"])
 def test_policy_forward_with_filters_matches_reference(ref, name):
-    torch.manual_seed(21)
-    Env = ref.TSPEnv if name == "tsp" else ref.CVRPEnv
-    env = Env(generator_params=dict(num_loc=20), check_solution=True)
-    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=1).eval()
-    W = {k: v.detach().clone() for k, v in pol.state_dict().items()}
-    td0 = env.generator(batch_size=[16])
-    inst = {k: td0[k].clone() for k in td0.keys()}
+    inst, want, W = golden_case(ref, f"filters_{name}")
     with torch.inference_mode():
         torch.manual_seed(9)
-        out = pol(env.reset(td0.clone()), env, phase="train", decode_type="sampling", top_k=5, top_p=0.9)
-        torch.manual_seed(9)
         o = O.policy_forward(W, name, inst, decode_type="sampling", num_layers=1, top_k=5, top_p=0.9)
-    assert torch.equal(out["actions"], o["actions"])
-    torch.testing.assert_close(out["log_likelihood"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
+    assert torch.equal(want["actions"], o["actions"])
+    torch.testing.assert_close(want["ll"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
 
 
 @pytest.mark.parametrize("name,n", [("tsp", 12), ("cvrp", 11)])
 @pytest.mark.parametrize("beam_width,select_best", [(3, True), (4, False), (None, True)])
 def test_beam_search_matches_reference(ref, name, n, beam_width, select_best):
-    """utils/decoding.py:464-600 through the live ConstructivePolicy loop."""
-    torch.manual_seed(300 + n)
-    Env = ref.TSPEnv if name == "tsp" else ref.CVRPEnv
-    env = Env(generator_params=dict(num_loc=n), check_solution=True)
-    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=1).eval()
-    W = {k: v.detach().clone() for k, v in pol.state_dict().items()}
-    td0 = env.generator(batch_size=[5])
-    inst = {k: td0[k].clone() for k in td0.keys()}
+    """utils/decoding.py:464-600 through the reference's ConstructivePolicy loop."""
+    inst, want, W = golden_case(ref, f"beam_{name}{n}_{beam_width}_{select_best}")
     kw = {} if beam_width is None else {"beam_width": beam_width}
     with torch.inference_mode():
-        out = pol(env.reset(td0.clone()), env, phase="test", decode_type="beam_search", select_best=select_best, **kw)
         o = O.policy_forward(W, name, inst, decode_type="beam_search", num_layers=1, select_best=select_best, **kw)
-    assert torch.equal(out["actions"], o["actions"])
-    torch.testing.assert_close(out["reward"], o["reward"], rtol=1e-6, atol=0)
-    torch.testing.assert_close(out["log_likelihood"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
+    assert torch.equal(want["actions"], o["actions"])
+    torch.testing.assert_close(want["reward"], o["reward"], rtol=1e-6, atol=0)
+    torch.testing.assert_close(want["ll"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
 
 
 def test_generator_matches_reference(ref):
     for name, n in (("tsp", 50), ("cvrp", 50), ("cvrp", 100)):
-        Env = ref.TSPEnv if name == "tsp" else ref.CVRPEnv
-        env = Env(generator_params=dict(num_loc=n))
-        torch.manual_seed(1234)
-        td = env.generator(batch_size=[5])
+        _, want, _ = golden_case(ref, f"gen_{name}{n}")
         torch.manual_seed(1234)
         inst = O.generate_instances(name, 5, n)
+        assert want and set(inst) <= set(want), name
         for k in inst:
-            assert torch.equal(td[k], inst[k]), (name, k)
+            assert torch.equal(want[k], inst[k]), (name, k)
 
 
 @pytest.mark.parametrize("name,n", [("op", 20), ("op", 33), ("pctsp", 20), ("pctsp", 41), ("sdvrp", 20)])
 @pytest.mark.parametrize("decode_type", ["greedy", "sampling"])
 def test_sibling_env_policy_forward_matches_reference(ref, name, n, decode_type):
-    """The sibling envs (SURVEY.md 8f-4) on fresh seeds: the live reference policy (its own env, init / context / dynamic
-    embeddings) against the oracle's restatement -- actions bit for bit, rewards and log-likelihoods to 1e-5."""
-    import importlib
-
-    torch.manual_seed(2000 + n)
-    cls = {"op": "OPEnv", "pctsp": "PCTSPEnv", "sdvrp": "SDVRPEnv"}[name]
-    Env = getattr(importlib.import_module(f"rl4co.envs.routing.{name}.env"), cls)
-    gp = dict(num_loc=n, prize_distribution="dist") if name == "op" else dict(num_loc=n)  # see make_golden.make_env
-    env = Env(generator_params=gp, check_solution=True)
-    pol = ref.AttentionModelPolicy(env_name=name, num_encoder_layers=2).eval()
-    W = {k: v.detach().clone() for k, v in pol.state_dict().items()}
-    td0 = env.generator(batch_size=[8])
-    inst = {k: td0[k].clone() for k in td0.keys()}
+    """The sibling envs (SURVEY.md 8f-4): the reference policy (its own env, init / context / dynamic embeddings)
+    against the oracle's restatement -- actions bit for bit, rewards and log-likelihoods to 1e-5."""
+    inst, want, W = golden_case(ref, f"sibling_{name}{n}_{decode_type}")
     with torch.inference_mode():
         torch.manual_seed(5)
-        out = pol(env.reset(td0.clone()), env, phase="test", decode_type=decode_type)
-        torch.manual_seed(5)
         o = O.policy_forward(W, name, inst, decode_type=decode_type, num_layers=2)
-    assert torch.equal(out["actions"], o["actions"])
-    torch.testing.assert_close(out["reward"], o["reward"], rtol=1e-5, atol=1e-6)
-    torch.testing.assert_close(out["log_likelihood"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
+    assert torch.equal(want["actions"], o["actions"])
+    torch.testing.assert_close(want["reward"], o["reward"], rtol=1e-5, atol=1e-6)
+    torch.testing.assert_close(want["ll"], o["log_likelihood"], rtol=1e-5, atol=1e-5)
