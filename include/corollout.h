@@ -128,6 +128,15 @@ int co_check_tours(const int64_t* actions, const float* demand,
                    const float* vehicle_capacity, int32_t* bad_count, int B, int B_inst,
                    int N, int T, void* stream);
 
+/* TSPEnv.local_search (rl4co/envs/routing/tsp/env.py:184-188 -> tsp/local_search.py:16-81): 2-opt on each tour,
+ * best improvement per scan, bit for bit the reference's result.  locs [B,N,2] f32, tours_in / tours_out [B,N] int64
+ * (may alias; the input is read whole before a row is written), moves_out [B] int32 or NULL: moves applied per row,
+ * at most max_iterations (0 leaves every row unchanged).  A row holding a node index outside [0, N) is copied
+ * unchanged and gets moves_out = -1.  No N x N matrix: shared memory per CTA is 16 * N bytes. */
+#define CO_TWO_OPT_MAX_NODES 1024
+int co_tsp_two_opt(const float* locs, const int64_t* tours_in, int64_t* tours_out, int32_t* moves_out,
+                   int B, int N, int max_iterations, void* stream);
+
 /* ------------------------------------------------------------------ decoder, one step */
 
 /* Weights of the decoder path, device pointers, all float32, no biases

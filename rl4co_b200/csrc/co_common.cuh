@@ -67,6 +67,14 @@ __device__ __forceinline__ void warp_argmax(float& v, int& idx) {
   }
 }
 
+// Euclidean distance as sqrt(fma(dy, dy, dx * dx)): what torch's CPU reduction produces for the 2-norm of a
+// two-element difference (torch.norm, rl4co/utils/ops.py:93-100), so recorded reference distances are met bit for
+// bit.  Symmetric exactly: dist2(a, b) == dist2(b, a).
+__device__ __forceinline__ float dist2(float2 a, float2 b) {
+  const float dx = a.x - b.x, dy = a.y - b.y;
+  return sqrtf(fmaf(dy, dy, dx * dx));
+}
+
 // Philox4x32-10 (Salmon et al. 2011), used for CO_SELECT_SAMPLE_PHILOX.
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
   const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;

@@ -2,19 +2,13 @@
 //   co_op_step        <- rl4co/envs/routing/op/env.py:72-105 (_step incl. the trailing get_action_mask)
 //   co_op_action_mask <- op/env.py:140-155
 //   co_op_reward      <- op/env.py:157-165 (sum of the collected prizes)
-// One warp per instance row.  The 2-norm of a coordinate difference is sqrt(fma(dy, dy, dx * dx)) -- what torch's CPU
-// reduction produces for two elements (checked against torch.norm: the golden traces were recorded on the CPU), so the
-// recorded tour lengths and masks are reproduced bit for bit.
+// One warp per instance row.  Distances are co::dist2 (co_common.cuh), so the recorded tour lengths and masks are
+// reproduced bit for bit.
 #include "co_common.cuh"
 
 namespace co {
 
 constexpr int OP_ROWS_PER_CTA = 8;
-
-__device__ __forceinline__ float dist2(float2 a, float2 b) {
-  const float dx = a.x - b.x, dy = a.y - b.y;
-  return sqrtf(fmaf(dy, dy, dx * dx));
-}
 
 // get_action_mask: visited | depot re-entered | tour_length + dist(cur, n) > max_length[n]; the depot is always feasible
 __device__ __forceinline__ void op_mask_row(const float2* __restrict__ locs, const float* __restrict__ max_length,

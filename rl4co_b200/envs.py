@@ -268,6 +268,10 @@ class FusedEnvBase:
                 td = self.generator(batch_size)
         return TensorDictDataset(td)
 
+    def local_search(self, td: TensorDict, actions: torch.Tensor, **kwargs) -> torch.Tensor:
+        """rl4co/envs/common/base.py:228-232"""
+        raise NotImplementedError(f"Local is not implemented yet for {self.name} environment")
+
     @staticmethod
     def load_data(fpath, batch_size=[]):
         from .data import load_npz_to_tensordict
@@ -343,6 +347,24 @@ class FusedTSPEnv(FusedEnvBase):
         """tsp/env.py:158-164"""
         bad = native.check_tours(actions.contiguous(), td["locs"].shape[-2])
         assert bad == 0, "Invalid tour"
+
+    @staticmethod
+    def local_search(td: TensorDict, actions: torch.Tensor, max_iterations: int = 1000,
+                     num_threads: int | None = None) -> torch.Tensor:
+        """tsp/env.py:184-188 -> tsp/local_search.py:16-81: 2-opt (best improvement per scan) on every tour, in one
+        kernel (co_tsp_two_opt) on the tensors' GPU; the same tours as the reference, bit for bit.  Returns new int64
+        tours [B, N]; `actions` is not modified.  `num_threads` (the reference's numba thread count) is ignored."""
+        if "distances" in td.keys():
+            raise NotImplementedError("local_search: a precomputed td['distances'] matrix is not supported; "
+                                      "distances are computed from td['locs']")
+        locs = td["locs"]
+        if actions.dim() != 2 or locs.dim() != 3 or tuple(locs.shape) != (*actions.shape, 2):
+            raise ValueError(f"local_search: actions must be [B, N] and td['locs'] [B, N, 2], got "
+                             f"{tuple(actions.shape)} and {tuple(locs.shape)}")
+        if actions.shape[1] > native.TWO_OPT_MAX_NODES:
+            raise NotImplementedError(f"local_search: N={actions.shape[1]} above {native.TWO_OPT_MAX_NODES} nodes")
+        return native.tsp_two_opt(locs.to(torch.float32).contiguous(), actions.to(torch.int64).contiguous(),
+                                  max_iterations)
 
 
 class FusedCVRPEnv(FusedEnvBase):

@@ -22,7 +22,8 @@ INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.path.join(_HERE, "libcorollout.so")
 SOURCES = ["abi.cu", "env_kernels.cu", "decode_step.cu", "rollout.cu", "rollout_tsp.cu", "rollout_cvrp.cu", "rollout_ms_tsp.cu", "rollout_ms_cvrp.cu", "rollout_sdvrp.cu", "rollout_op.cu", "rollout_pctsp.cu", "gemm_tf32x3.cu",
            "encoder_mha.cu", "encoder_mha_tc.cu", "encoder_mha_tc2.cu", "encoder_mha_tc3.cu",
-           "ffn_fused.cu", "data_kernels.cu", "attn_train.cu", "norm_kernels.cu", "op_kernels.cu"]
+           "ffn_fused.cu", "data_kernels.cu", "attn_train.cu", "norm_kernels.cu", "op_kernels.cu",
+           "two_opt.cu"]
 HEADERS = ["co_common.cuh", "rollout_impl.cuh", "rollout_ms_impl.cuh"]
 
 CO_OK = 0
@@ -35,6 +36,7 @@ ROLLOUT_ENVS = ("tsp", "cvrp", "sdvrp", "op", "pctsp")
 SELECT_GREEDY, SELECT_SAMPLE_NOISE, SELECT_EVALUATE, SELECT_SAMPLE_PHILOX = 0, 1, 2, 3
 ROLLOUT_FORCED_START = 1
 EMBED_DIM, NUM_HEADS = 128, 8
+TWO_OPT_MAX_NODES = 1024  # CO_TWO_OPT_MAX_NODES
 
 EXPORTS = [
     "co_version", "co_last_error_string", "co_device_sm_count", "co_tsp_step", "co_cvrp_action_mask",
@@ -42,6 +44,7 @@ EXPORTS = [
     "co_cache_width", "co_rollout_max_nodes", "co_rollout", "co_reward_stats", "co_split_tf32", "co_gemm_tf32x3", "co_encoder_mha",
     "co_ffn_fused", "co_ffn_tile_weights", "co_ffn_tiled_weight_floats", "co_generate_uniform", "co_generate_demand", "co_dihedral8",
     "co_sdvrp_step", "co_sdvrp_action_mask", "co_attn_fwd", "co_attn_bwd", "co_instance_norm", "co_op_step", "co_op_action_mask", "co_op_reward", "co_pctsp_step", "co_pctsp_action_mask",
+    "co_tsp_two_opt",
 ]
 
 
@@ -149,6 +152,7 @@ def lib() -> ctypes.CDLL:
     L.co_pctsp_action_mask.argtypes = [c_void_p] * 3 + [c_int, c_int, c_void_p]
     L.co_pctsp_step.argtypes = [c_void_p] * 11 + [c_int, c_int, c_void_p]
     L.co_op_reward.argtypes = [c_void_p] * 3 + [c_int, c_int, c_int, c_void_p]
+    L.co_tsp_two_opt.argtypes = [c_void_p] * 4 + [c_int, c_int, c_int, c_void_p]
     L.co_instance_norm.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_long, c_int, c_float, c_void_p]
     L.co_attn_fwd.argtypes = [POINTER(AttnArgs), c_void_p]
     L.co_attn_bwd.argtypes = [POINTER(AttnArgs), c_void_p]
@@ -341,6 +345,24 @@ def op_reward(prize, actions):
     out = torch.empty(B, dtype=F32, device=actions.device)
     _check(lib().co_op_reward(_ptr(prize.contiguous(), F32, "prize"), _ptr(actions, I64, "actions"), _ptr(out, F32, "reward"),
                               B, prize.shape[1], T, _stream()), "co_op_reward")
+    return out
+
+
+@_on_device_of_first_tensor
+def tsp_two_opt(locs, tours, max_iterations, moves=None):
+    """co_tsp_two_opt (tsp/local_search.py:16-81): 2-opt on tours [B, N] int64 over locs [B, N, 2] -> a new [B, N] int64
+    tensor; the input is not modified.  `moves` ([B] int32), if given, receives the moves applied per row, or -1 for a
+    row with a node index outside [0, N), which is returned unchanged.  max_iterations <= 0 changes nothing."""
+    if tours.dim() != 2 or tuple(locs.shape) != (*tours.shape, 2):
+        raise ValueError(f"tours must be [B, N] and locs [B, N, 2], got {tuple(tours.shape)} and {tuple(locs.shape)}")
+    B, N = tours.shape
+    if moves is not None and tuple(moves.shape) != (B,):
+        raise ValueError(f"moves must be [{B}], got {tuple(moves.shape)}")
+    out = torch.empty_like(tours)
+    args = (_ptr(locs, F32, "locs"), _ptr(tours, I64, "tours"), _ptr(out, I64, "tours_out"), _ptr(moves, I32, "moves"))
+    if B == 0:
+        return out
+    _check(lib().co_tsp_two_opt(*args, B, N, max(0, min(int(max_iterations), 2**31 - 1)), _stream()), "co_tsp_two_opt")
     return out
 
 

@@ -58,3 +58,16 @@ AT.self_attention_packed(qkv).sum().backward()
 native.instance_norm(torch.randn(9, 100, 128, device=dev), torch.ones(128, device=dev), torch.zeros(128, device=dev))
 torch.cuda.synchronize()
 print("attention / norm ok")
+# 2-opt local search: random tours to convergence, a row with an out-of-range node, a capped TSP-1000 run
+from rl4co_b200.envs import FusedTSPEnv
+from rl4co_b200.tensordict import TensorDict
+
+for B, n, iters in ((64, 50, 1000), (2, 1000, 20)):
+    locs = torch.rand(B, n, 2, device=dev)
+    tours = torch.rand(B, n, device=dev).argsort(1)
+    tours[0, 1] = n
+    moves = torch.empty(B, dtype=torch.int32, device=dev)
+    out = native.tsp_two_opt(locs, tours, iters, moves=moves)
+    FusedTSPEnv.local_search(TensorDict({"locs": locs[1:]}, batch_size=[B - 1]), tours[1:], iters)
+    torch.cuda.synchronize()
+    print("two_opt", n, "ok", moves.tolist()[:4])
